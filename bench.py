@@ -43,7 +43,41 @@ def parse():
     ap.add_argument("--e2e-pipelines", type=int, default=2,
                     help="independent encoder/decoder handle pairs streaming side by side in the end-to-end leg (each pair = two host "
                          "threads; a second pair fills the copy-engine bubbles between the batches of the first)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last step computed to DIR/*.npy (rank 0): a seeded sample of the "
+                         "decoded points, the encoded size of every frame and a seeded sample of the encoded bytes")
     return ap.parse_args()
+
+
+DUMP_POINTS = 1 << 20       # decoded points sampled over the whole batch (16 MB as float32)
+DUMP_BLOB_BYTES = 24 << 20  # encoded bytes sampled over the batch (as float32: at most 24 MB, 40 MB in all)
+
+
+def dump_outputs(out_dir, d_out, d_blob, sizes):
+    """The arrays the last timed step handed its caller: the decoded clouds (float32 x, y, z, intensity) and the encoded
+    blobs. Both are sampled at positions drawn from fixed seeds, so two builds of the library can be compared output for
+    output; the blobs' bytes are stored as float32 values 0..255 and their sizes as float64."""
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    F = len(d_out)
+    pick = np.sort(np.random.default_rng(0).choice(F * POINTS, size=min(DUMP_POINTS, F * POINTS), replace=False))
+    frame, point = pick // POINTS, pick % POINTS
+    pts = np.empty((pick.size, 4), dtype=np.float32)
+    for k in range(F):
+        sel = frame == k
+        if sel.any():
+            idx = torch.from_numpy(point[sel]).to(d_out[k].device)
+            pts[sel] = d_out[k].view(torch.float32).view(POINTS, 4)[idx].cpu().numpy()
+    rng = np.random.default_rng(1)
+    per_frame = max(1, min(1 << 15, DUMP_BLOB_BYTES // (4 * F)))
+    blob_bytes = np.empty((F, per_frame), dtype=np.float32)
+    for k in range(F):
+        pos = np.sort(rng.integers(0, int(sizes[k]), per_frame))
+        blob_bytes[k] = d_blob[k][torch.from_numpy(pos).to(d_blob[k].device)].cpu().numpy()
+    np.save(os.path.join(out_dir, "decoded_points.npy"), pts)
+    np.save(os.path.join(out_dir, "decoded_points_index.npy"), pick.astype(np.float64))
+    np.save(os.path.join(out_dir, "blob_sizes.npy"), np.asarray(sizes, dtype=np.float64))
+    np.save(os.path.join(out_dir, "blob_bytes.npy"), blob_bytes)
 
 
 class ClockSampler:
@@ -271,6 +305,8 @@ def main():
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     if args.impl == "reference":
+        if args.dump_outputs:
+            raise SystemExit("bench.py: --dump-outputs needs --impl ours (the reference leg times its passes inside the reference library)")
         run_reference(args, rank, world)
         return
 
@@ -366,6 +402,11 @@ def main():
     clocks = sampler.stop() if rank == 0 else None
     enc.sync()
     dec.sync()
+    if args.dump_outputs and rank == 0:
+        # the encoded sizes of the last timed launch, as the encoder left them on the device (uint64 per frame)
+        last = type("DeviceSizes", (), {"__cuda_array_interface__": {"shape": (F,), "typestr": "<i8", "data": (enc.sizes_device_ptr(), False),
+                                                                      "version": 3}})()
+        dump_outputs(args.dump_outputs, d_out, d_blob, torch.as_tensor(last, device=dev).cpu().numpy())
     elapsed_ms = t_start.elapsed_time(t_end)
     enc_ms = float(np.mean([e[0].elapsed_time(e[1]) for e in evs]))
     dec_ms = float(np.mean([e[1].elapsed_time(e[2]) for e in evs]))

@@ -2,12 +2,15 @@
 
 * ``RefOracle``  — oracle/_ref/libcloudini_ref.so: the UNMODIFIED reference compiled in place (oracle/build_ref.sh).
 * ``PortOracle`` — oracle/_build/libcloudini_oracle.so: the plain-C restatement (oracle/cloudini_oracle.c).
+* ``RecordedRef`` — the reference's answers to the tests' calls (tests/golden/ref_answers.npz), where oracle/_ref is absent.
 
 Only tests/, __graft_entry__.smoke() and bench.py's cpu_baseline / --impl reference legs import this module.
 """
 from __future__ import annotations
 
 import ctypes as C
+import hashlib
+import inspect
 import os
 import subprocess
 
@@ -287,3 +290,226 @@ class PortOracle:
 def best_oracle():
     """The reference itself when its .so is available, else the C port."""
     return RefOracle() if have_ref() else PortOracle()
+
+
+# ---- the reference's answers, recorded -------------------------------------------------------------------------------
+# The compiled reference exists only where its source tree does. Its answers to the calls the tests make are recorded
+# into tests/golden/ref_answers.npz by running the tests against it, on a GPU for the `gpu` ones
+# (CLDN_REF_RECORD=$PWD/tests/golden/ref_answers.npz python -m pytest tests; new answers are merged into the file),
+# and replayed by RecordedRef everywhere else. A call is keyed by a digest of its arguments; an answer up to SMALL_ANSWER bytes is stored
+# whole, a larger one as its digest, and the replay then rebuilds the bytes with a local implementation (the C port, or
+# this library) and hands them out only if they hash to the reference's digest.
+ANSWERS = os.path.join(os.path.dirname(HERE), "tests", "golden", "ref_answers.npz")
+SMALL_ANSWER = 1024
+_REPLAYED = ("max_compressed_size", "encode", "header", "decode_header", "decode", "decode_payload", "viz_preprocess",
+             "ros_describe", "ros_compress", "ros_decompress")
+_OUT_ARG = {"decode": 1, "decode_payload": 2}   # the argument these methods fill in place
+
+
+def _digest(data: bytes) -> bytes:
+    return hashlib.sha256(data).digest()[:16]
+
+
+def _call_key(name: str, bound) -> bytes:
+    h = hashlib.sha256(name.encode())
+    for a in bound:
+        if isinstance(a, cb.EncodingInfo):
+            part = b"info:%d:" % int(a.version) + _yaml(a)
+        elif isinstance(a, (bytes, bytearray, memoryview, np.ndarray)):
+            part = b"buf:" + _u8(a).tobytes()
+        elif isinstance(a, dict):
+            part = repr(sorted((k, float(v)) for k, v in a.items())).encode()
+        else:
+            part = repr(a).encode()
+        h.update(len(part).to_bytes(8, "little") + part)
+    return h.digest()[:16]
+
+
+def _bind(name: str, args, kwargs):
+    sig = inspect.signature(getattr(RefOracle, name))
+    b = sig.bind(None, *args, **kwargs)
+    b.apply_defaults()
+    return list(b.arguments.values())[1:]
+
+
+def _answer_parts(result):
+    """A return value as (tag, bytes) parts: b bytes, a array, s str, i int, y EncodingInfo."""
+    out = []
+    for r in (result if isinstance(result, tuple) else (result,)):
+        if isinstance(r, (bytes, bytearray)):
+            out.append((b"b", bytes(r)))
+        elif isinstance(r, np.ndarray):
+            out.append((b"a", _u8(r).tobytes()))
+        elif isinstance(r, str):
+            out.append((b"s", r.encode()))
+        elif isinstance(r, cb.EncodingInfo):
+            out.append((b"y", b"%d:" % int(r.version) + _yaml(r)))
+        else:
+            out.append((b"i", str(int(r)).encode()))
+    return out
+
+
+def _pack(parts) -> bytes:
+    return b"".join(len(p).to_bytes(4, "little") + p for p in parts)
+
+
+def _unpack(raw: bytes):
+    parts, pos = [], 0
+    while pos < len(raw):
+        n = int.from_bytes(raw[pos:pos + 4], "little")
+        parts.append(raw[pos + 4:pos + 4 + n])
+        pos += 4 + n
+    return parts
+
+
+def _stored(result=None, error=None) -> bytes:
+    """What the answer file keeps of one answer: b"E" + message, or b"R" + per part its tag (upper case = digest only)."""
+    if error is not None:
+        return b"E" + str(error).encode()
+    parts = []
+    for tag, data in _answer_parts(result):
+        parts += [tag.upper(), _digest(data)] if len(data) > SMALL_ANSWER else [tag, data]
+    return b"R" + _pack(parts)
+
+
+def _load_answers(path):
+    if not os.path.exists(path):
+        return {}
+    z = np.load(path)
+    keys, offs, blob = z["keys"], z["offsets"], z["answers"].tobytes()
+    return {keys[i].tobytes(): blob[offs[i]:offs[i + 1]] for i in range(len(keys))}
+
+
+def _save_answers(path, answers):
+    keys = sorted(answers)
+    offs = np.zeros(len(keys) + 1, dtype=np.int64)
+    offs[1:] = np.cumsum([len(answers[k]) for k in keys])
+    np.savez_compressed(path, keys=np.frombuffer(b"".join(keys), dtype=np.uint8).reshape(-1, 16),
+                        offsets=offs, answers=np.frombuffer(b"".join(answers[k] for k in keys), dtype=np.uint8))
+
+
+class RecordingRef(RefOracle):
+    """RefOracle that also keeps every answer it gives; save() merges them into an answer file."""
+
+    def __init__(self, path):
+        super().__init__()
+        self.path, self.answers = path, {}
+
+    def __getattribute__(self, name):
+        real = super().__getattribute__(name)
+        if name not in _REPLAYED:
+            return real
+
+        def call(*args, **kwargs):
+            key = _call_key(name, _bind(name, args, kwargs))
+            try:
+                result = real(*args, **kwargs)
+            except RuntimeError as e:
+                self.answers[key] = _stored(error=e)
+                raise
+            self.answers[key] = _stored(result)
+            return result
+        return call
+
+    def save(self):
+        answers = _load_answers(self.path)
+        answers.update(self.answers)
+        _save_answers(self.path, answers)
+
+
+class _LibraryAnswers:
+    """This library's own calls that compute what a RefOracle method returns (the GPU codec, host-side stage 2)."""
+
+    def encode(self, info, cloud, write_header=True, cap=None):
+        return cb.PointcloudEncoder(info).encode(cloud, write_header)
+
+    def decode(self, blob, out):
+        info, hdr = cb.DecodeHeader(blob)
+        cb.PointcloudDecoder().decode(info, bytes(blob)[hdr:], out)
+        return out
+
+    def ros_compress(self, msg, profile=None, default_resolution=None, viz=False, encoding_opt=1, compression_opt=0, version=5):
+        from cloudini_b200 import ros
+        return ros.convert_message(msg, profile or {}, default_resolution, viz, cb.EncodingOptions(encoding_opt),
+                                   cb.CompressionOption(compression_opt), version)
+
+    def ros_decompress(self, msg, capacity):
+        from cloudini_b200 import ros
+        return ros.convertCompressedCloudToPointCloud2(ros.getDeserializedPointCloudMessage(msg))
+
+
+class RecordedRef:
+    """The reference's recorded answers (tests/golden/ref_answers.npz) behind RefOracle's methods. A call the
+    reference was never asked, or an answer no local implementation reproduces, fails the calling test."""
+    kind = "reference (recorded answers)"
+
+    def __init__(self, path=ANSWERS):
+        self.answers = _load_answers(path)
+        if not self.answers:
+            raise RuntimeError(f"{path}: no recorded answers of the reference")
+        self._makers = [PortOracle(), _LibraryAnswers()]
+
+    def __getattr__(self, name):
+        if name not in _REPLAYED:
+            raise AttributeError(name)
+
+        def call(*args, **kwargs):
+            bound = _bind(name, args, kwargs)
+            stored = self.answers.get(_call_key(name, bound))
+            if stored is None:
+                raise AssertionError(f"ref.{name}: the reference was never asked this (tests/golden/ref_answers.npz has no "
+                                     "answer for these arguments)")
+            if stored[:1] == b"E":
+                raise RuntimeError(stored[1:].decode("utf-8", "replace"))
+            parts = _unpack(stored[1:])
+            want = list(zip(parts[0::2], parts[1::2]))
+            if all(tag.islower() for tag, _ in want):
+                return self._result(name, bound, want)
+            for maker in self._makers:
+                if not hasattr(maker, name):
+                    continue
+                args2 = [np.array(a, copy=True) if isinstance(a, np.ndarray) else a for a in bound]
+                try:
+                    result = getattr(maker, name)(*args2)
+                except Exception:  # noqa: BLE001 - a maker that cannot run here (no GPU) or disagrees is not the answer
+                    continue
+                got = _answer_parts(result)
+                if len(got) == len(want) and all(t == wt.lower() and (d == wd if wt.islower() else _digest(d) == wd)
+                                                 for (t, d), (wt, wd) in zip(got, want)):
+                    if name in _OUT_ARG:
+                        _u8(bound[_OUT_ARG[name]])[:] = _u8(result)
+                        return bound[_OUT_ARG[name]]
+                    return result
+            raise AssertionError(f"ref.{name}: no local implementation reproduces the reference's recorded answer")
+        return call
+
+    def _result(self, name, bound, want):
+        vals = []
+        for tag, data in want:
+            if tag == b"b":
+                vals.append(data)
+            elif tag == b"a":
+                vals.append(np.frombuffer(data, dtype=np.uint8).copy())
+            elif tag == b"s":
+                vals.append(data.decode())
+            elif tag == b"y":
+                ver, text = data.split(b":", 1)
+                info = cb.EncodingInfoFromYAML(text.decode())
+                info.version = int(ver)
+                vals.append(info)
+            else:
+                vals.append(int(data))
+        if name in _OUT_ARG:
+            out = bound[_OUT_ARG[name]]
+            _u8(out)[:] = vals[0]
+            return out
+        return tuple(vals) if len(vals) > 1 else vals[0]
+
+
+def reference_oracle():
+    """The compiled reference where it is available (recording its answers into the file CLDN_REF_RECORD names, if
+    set), else its recorded answers."""
+    if have_ref():
+        path = os.environ.get("CLDN_REF_RECORD")
+        return RecordingRef(path) if path else RefOracle()
+    return RecordedRef()

@@ -44,11 +44,13 @@ def port(lib_built):
 
 @pytest.fixture(scope="session")
 def ref(lib_built):
-    from oracle.client import RefOracle, build_ref, have_ref
+    """The compiled reference where it can be built, else its answers recorded in tests/golden/ref_answers.npz."""
+    from oracle.client import RecordingRef, build_ref, reference_oracle
     build_ref()
-    if not have_ref():
-        pytest.skip("oracle/_ref/libcloudini_ref.so unavailable (no /root/reference here and no prebuilt copy)")
-    return RefOracle()
+    r = reference_oracle()
+    yield r
+    if isinstance(r, RecordingRef):
+        r.save()
 
 
 @pytest.fixture(scope="session")
